@@ -184,7 +184,7 @@ def bench_ours(args, cfg, rank, local, world):
         c = cam["c"]
         out = C.rasterize_gaussians(bg, means3D, feats, E, opac, scales, rots, 1.0, E, cam["view"], cam["proj"],
                                     c.tanfovx, c.tanfovy, c.cx, c.cy, H, W, shs, 3, cam["pos"], False, True, False)
-        stats["R"] = out[0]; stats["radii"] = out[9]
+        stats["R"] = out[0]; stats["radii"] = out[9]; stats["out"] = out
         C.rasterize_gaussians_backward(bg, means3D, feats, out[9], E, scales, rots, 1.0, E, cam["view"], cam["proj"],
                                        c.tanfovx, c.tanfovy, dcot["color"], dcot["opacity"], dcot["depth"],
                                        dcot["feature"], shs, 3, cam["pos"], out[10], out[0], out[11], out[12],
@@ -244,6 +244,8 @@ def bench_ours(args, cfg, rank, local, world):
     ms, stage, launches = timed(step_resident, args.steps, args.warmup, profile=True)
     blocks = stats["blocks"]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats["out"], bucket.views)
     value = world * args.steps / (ms / 1e3)
 
     # ---- e2e: public API (module + autograd), per-step host inputs from pinned memory -------
@@ -307,7 +309,7 @@ def bench_ours(args, cfg, rank, local, world):
         loss_host[i % 64:i % 64 + 1].copy_(loss.detach().reshape(1), non_blocking=True)
 
     leaf_bucket = rdist.LeafGradBucket([params[k] for k in (0, 1, 3, 4, 5)], dev, symmetric=exchange_kind == "p2p") if factored else None
-    e_steps = max(50, args.steps)
+    e_steps = args.steps
     # (1) the path an UNCHANGED caller of the reference surface gets: synchronous instance count (one host wait per forward,
     #     like the reference's own cudaMemcpy at rasterizer_impl.cu:291).  Its warm-up also teaches the deferred path the counts.
     set_deferred_count(False)
@@ -363,6 +365,32 @@ def bench_ours(args, cfg, rank, local, world):
                          "step_alg_bytes": step_alg, "step_frac_of_peak": step_alg / (ms / args.steps * 1e-3) / 1e9 / peak},
         }
     return res
+
+
+DUMP_ROWS = 32768         # per-Gaussian outputs: a fixed, seeded sample of this many Gaussians (rows)
+
+
+def dump_outputs(outdir, out, grads):
+    """What the timed step returned in its last step, as <outdir>/<name>.npy: the rendered images and the per-pixel
+    contributor counts whole, the per-Gaussian outputs (radii, weights, parameter gradients) on a seeded sample of
+    DUMP_ROWS Gaussians (their indices in sample_rows.npy).  Float32 as computed; integers as float64 (exact)."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    P = out[9].shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(P, size=min(P, DUMP_ROWS), replace=False))
+    rows_dev = torch.from_numpy(rows).to(out[9].device)
+    arrays = {"num_rendered": np.array([int(out[0])], np.float64), "sample_rows": rows.astype(np.float64),
+              "n_contrib": out[1].cpu().numpy().astype(np.float64), "radii": out[9][rows_dev].cpu().numpy().astype(np.float64)}
+    for i, name in enumerate(("color", "opacity", "depth", "feature", "normal", "surface_xyz", "weights"), start=2):
+        t = out[i] if name != "weights" else out[i][rows_dev]
+        arrays[name] = t.float().cpu().numpy()
+    for name, t in grads.items():
+        arrays["grad_" + name] = t[rows_dev].float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit(f"--dump-outputs: {total / 2**20:.1f} MB exceeds 64 MB at this configuration")
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
 
 
 def cpu_baseline_sample(cfg, seconds_budget=25.0):
@@ -480,7 +508,7 @@ def main():
 
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 30 for --workload stage2)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--P", type=int, default=None)
@@ -495,7 +523,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--exchange", default="auto", choices=["auto", "p2p", "factored", "dense"],
                     help="N > 1: gradient exchange per step (DESIGN.md section 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (headline workload, ours)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "headline"):
+        ap.error("--dump-outputs applies to the headline workload of --impl ours")
+    if args.steps is None:
+        args.steps = 30 if args.workload == "stage2" else 200     # a stage-2 step is ~10x a headline step
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     args.warmup = max(args.warmup, 3)
     cfg = dict(HEADLINE)
     for k in ("P", "W", "H", "S"):
@@ -509,8 +545,6 @@ def main():
         for k in ("P", "W", "H", "N"):
             if getattr(args, k) is not None:
                 cfg2[k] = getattr(args, k)
-        if args.steps == 200:
-            args.steps = 30                     # a stage-2 step is ~10x a headline step
         if args.impl == "reference":
             if rank == 0:
                 emit(bench_stage2.run_reference(args, cfg2, rank, local, world))

@@ -54,7 +54,7 @@ if [ ! -f "$OUT/ext/r3dg_rasterization/_C.so" ]; then
 fi
 
 if [ ! -f "$OUT/ext/bvh_tracing/_C.so" ]; then
-  echo "[build_ref_ext] bvh_tracing._C (construct.cu: the one-line `-> aabb_type` patched copy, SURVEY §8c-addendum)"
+  echo "[build_ref_ext] bvh_tracing._C (construct.cu: the one-line '-> aabb_type' patched copy, SURVEY §8c-addendum)"
   sed '166s/rhs)[[:space:]]*{/rhs) -> aabb_type {/' "$BVH/src/construct.cu" > "$OUT/construct_patched.cu"
   diff "$BVH/src/construct.cu" "$OUT/construct_patched.cu" || true
   $NVCC $ARCH -O3 $TORCHISH -DTORCH_EXTENSION_NAME=_C --expt-extended-lambda -I"$BVH/include" $TORCH_INC -Xcompiler -fPIC \

@@ -1,4 +1,5 @@
 """Shared test utilities: seeded cases, conversions, comparison helpers."""
+import hashlib
 import os
 import sys
 
@@ -52,6 +53,105 @@ def max_rel_above_floor(a, b, floor=1e-6):
     if not m.any():
         return 0.0
     return float((np.abs(a - b)[m] / np.abs(b)[m]).max())
+
+
+def digest(a):
+    """sha256 of an integer / boolean array's values (as int64): stands in for a bit-exact comparison with a
+    stored reference array that is too large to keep."""
+    a = npy(a) if torch.is_tensor(a) else np.asarray(a)
+    return hashlib.sha256(np.ascontiguousarray(a, dtype=np.int64).tobytes()).hexdigest()
+
+
+def spread(a, rows=None, k=128):
+    """k evenly spaced elements of `a` (of its rows `rows` only, when given), flattened, as float32: a fixed
+    sample that stands in for a stored reference array that is too large to keep."""
+    a = npy(a) if torch.is_tensor(a) else np.asarray(a)
+    a = a.reshape(a.shape[0], -1)[rows].reshape(-1) if rows is not None else a.reshape(-1)
+    if a.size == 0:
+        return np.zeros(0, np.float32)
+    return a[np.linspace(0, a.size - 1, min(k, a.size)).astype(np.int64)].astype(np.float32)
+
+
+def summarize(prefix, a, rows=None):
+    """What a golden file keeps of a float array: a fixed sample (`spread`), its full L2 norm and max-abs."""
+    a = np.asarray(npy(a) if torch.is_tensor(a) else a, np.float64)
+    return {prefix: spread(a, rows), prefix + "_l2": np.float64(np.linalg.norm(a)),
+            prefix + "_maxabs": np.float64(np.abs(a).max(initial=0.0))}
+
+
+def assert_close_to_summary(g, prefix, a, rows=None, max_abs=None, rel=None):
+    """`a` against a stored `summarize` record.  max_abs: every sampled element within it, and the full L2 norms
+    within max_abs * sqrt(n) (what a full max-abs bound implies); rel: relative L2 error of the sample below it,
+    and the full L2 norms within rel (what a full relative L2 bound implies)."""
+    a = np.asarray(npy(a) if torch.is_tensor(a) else a, np.float64)
+    ref = g[prefix]
+    s = spread(a, rows, k=ref.size)
+    assert s.shape == ref.shape, (prefix, s.shape, ref.shape)
+    dn = abs(float(np.linalg.norm(a)) - float(g[prefix + "_l2"]))
+    if max_abs is not None:
+        assert np.abs(s - ref).max(initial=0.0) <= max_abs, (prefix, np.abs(s - ref).max())
+        assert dn <= max_abs * np.sqrt(a.size), (prefix, dn)
+    if rel is not None:
+        assert rel_l2(s, ref) < rel, (prefix, rel_l2(s, ref))
+        assert dn < rel * float(g[prefix + "_l2"]), (prefix, dn)
+
+
+def summarize_visibility(prefix, vis, step=8):
+    """What a golden file keeps of a visibility tensor [P, ...]: for every `step`-th Gaussian, which rays are blocked
+    (bit-packed) and a fixed sample of the values."""
+    v = np.asarray(npy(vis) if torch.is_tensor(vis) else vis)[::step].reshape(-1)
+    return {prefix + "_blocked": np.packbits(v == 0), prefix + "_values": spread(v, k=2048)}
+
+
+def assert_visibility_close(g, prefix, vis, max_flips, max_abs, step=8):
+    """`vis` against a `summarize_visibility` record: the share of rays whose blocked / visible outcome differs (the
+    T < 0.9 cliff) at most max_flips, the sampled values of rays on the same side within max_abs."""
+    v = np.asarray(npy(vis) if torch.is_tensor(vis) else vis)[::step].reshape(-1)
+    blocked = np.unpackbits(g[prefix + "_blocked"], count=v.size).astype(bool)
+    flips = float((blocked != (v == 0)).mean())
+    s, ref = spread(v, k=2048), g[prefix + "_values"]
+    same = (s == 0) == (ref == 0)
+    err = float(np.abs(s - ref)[same].max(initial=0.0))
+    assert flips <= max_flips and err <= max_abs, (prefix, flips, err)
+    return flips, err
+
+
+_KINDS = {"float32": "f4", "uint8": "u1", "str": "U64"}
+
+
+def pack_golden_case(key, rec):
+    """One case of a golden file that holds several, as a few npz entries (an npz of many small arrays is mostly zip
+    headers): the values of all arrays of one kind (float32, uint8, str, float64 for the rest) concatenated, and an
+    index of `name kind offset shape` lines.  GoldenCase reads it back."""
+    groups, index = {}, []
+    for name, v in rec.items():
+        v = np.asarray(v)
+        kind = "str" if v.dtype.kind == "U" else v.dtype.name if v.dtype.name in _KINDS else "float64"
+        arrs = groups.setdefault(kind, [])
+        index.append(f"{name} {kind} {sum(a.size for a in arrs)} {','.join(map(str, v.shape))}")
+        arrs.append(v.reshape(-1).astype(_KINDS.get(kind, "f8")))
+    return {f"{key}.index": np.array(index), **{f"{key}.{k}": np.concatenate(a) for k, a in groups.items()}}
+
+
+class GoldenCase:
+    """One case of a golden file written with pack_golden_case: a mapping name -> array."""
+
+    def __init__(self, path, key):
+        z = np.load(path)
+        assert f"{key}.index" in z.files, \
+            f"{os.path.basename(path)} has no case {key}: regenerate it with tests/golden/make_golden_refparity.py"
+        self.items = {}
+        for line in z[f"{key}.index"]:
+            name, kind, off, shape = str(line).split(" ")
+            shape = tuple(int(x) for x in shape.split(",") if x)
+            flat = z[f"{key}.{kind}"]
+            self.items[name] = flat[int(off):int(off) + int(np.prod(shape))].reshape(shape)
+
+    def __getitem__(self, name):
+        return self.items[name]
+
+    def __contains__(self, name):
+        return name in self.items
 
 
 def inverse_covariance(scales, rotations):

@@ -1,25 +1,48 @@
-"""The drop-in boundary, executed for real (SURVEY.md §8b): the reference's OWN wrapper files
-(gaussian_renderer/r3dg_rasterization.py, bvh/__init__.py — git-ignored copies under oracle/_ref/py made
-by oracle/build_ref_ext.sh) are loaded by path twice: once over the reference's own pybind modules
-(oracle/_ref/ext: rasterize_points.cu / bvh.cu glue + its kernels, built for sm_100) and once over this
-repo's `dropin/` packages.  Same inputs, same wrapper code, two back ends: outputs and gradients must agree
-to the north_star tolerances.  Also: the full visibility bake (own tree + in-kernel sampling + own trace)
-against the reference's bake (its tree + PyTorch sampling + its trace), and the sampling kernel against the
-reference's own `fibonacci_sphere_sampling`."""
+"""The drop-in boundary (SURVEY.md §8b): this repo's `dropin/` packages against the reference's own code path on the
+same seeded inputs — its Python wrapper files (gaussian_renderer/r3dg_rasterization.py, bvh/__init__.py) over its own
+pybind modules (rasterize_points.cu / bvh.cu glue + its kernels, built for sm_100).  What the reference computed is
+stored in tests/golden/refparity_dropin.npz (tests/golden/make_golden_refparity.py): sha256 of the arrays compared
+bit-exactly, a fixed sample and the full L2 norm of the others.  Outputs and gradients must agree to the north_star
+tolerances.  Also: the full visibility bake (own tree + in-kernel sampling + own trace) against the reference's bake
+(its tree + PyTorch sampling + its trace), and the sampling kernel against the reference's own
+`fibonacci_sphere_sampling`."""
+import os
+import sys
+
 import numpy as np
 import pytest
 import torch
 
-from helpers import case_inputs, npy, rel_l2
+from helpers import (GOLDEN, ROOT, GoldenCase, assert_close_to_summary, assert_visibility_close, case_inputs, digest,
+                     npy, spread)
 
 pytestmark = pytest.mark.gpu
+REF_DROPIN = os.path.join(GOLDEN, "refparity_dropin.npz")
+WRAPPER_IMAGES = ("color", "opacity", "depth", "feature", "normal", "surface_xyz")
+RAYTRACER_P = 30_000
+SAMPLING_N = (24, 32, 384)
 
 
-def _need(which):
-    from oracle import ref_gpu
-    if not ref_gpu.ext_available(which):
-        pytest.skip(f"oracle/_ref/ext ({which}) not built — run oracle/build_ref_ext.sh in the build container")
-    return ref_gpu
+def dropin(name):
+    """The drop-in package `name` (r3dg_rasterization / bvh_tracing) as a caller that put dropin/ on its path sees it."""
+    import importlib
+    path = os.path.join(ROOT, "dropin")
+    if path not in sys.path:
+        sys.path.insert(0, path)
+    return importlib.import_module(name)
+
+
+def wrapper_case(P, W, H, S):
+    sc, cam = case_inputs(P, W, H, S, view=4, center_shift=True)
+    g = torch.Generator().manual_seed(3)
+    return sc, cam, torch.tensor([0.3, 0.1, 0.7]), [torch.randn(c, H, W, generator=g) for c in (3, 1, 1, S)]
+
+
+def sampling_normals():
+    g = torch.Generator().manual_seed(1)
+    nrm = torch.nn.functional.normalize(torch.randn(50_000, 3, generator=g), dim=-1).cuda()
+    nrm[0] = torch.tensor([0.0, 0.0, -1.0]); nrm[1] = torch.tensor([0.0, 0.0, 1.0])      # the -I fallback and the identity
+    return nrm
 
 
 def _render_through_wrapper(mod, sc, cam, S, bg, cots):
@@ -50,25 +73,21 @@ def _render_through_wrapper(mod, sc, cam, S, bg, cots):
 
 
 @pytest.mark.parametrize("P,W,H,S", [(60_000, 400, 304, 16), (300_000, 800, 800, 5)], ids=["60k-S16", "300k-S5"])
-def test_reference_wrapper_runs_unmodified_over_dropin(P, W, H, S):
-    ref_gpu = _need("raster")
-    ours = ref_gpu.load_reference_wrapper("raster", "dropin")
-    theirs = ref_gpu.load_reference_wrapper("raster", "ref")
-    assert "relightable3dgaussian_b200" in ours._C_origin and "oracle/_ref/ext" in theirs._C_origin
-    sc, cam = case_inputs(P, W, H, S, view=4, center_shift=True)
-    bg = torch.tensor([0.3, 0.1, 0.7])
-    g = torch.Generator().manual_seed(3)
-    cots = [torch.randn(c, H, W, generator=g) for c in (3, 1, 1, S)]
-    ro, rg = _render_through_wrapper(theirs, sc, cam, S, bg, cots)
-    oo, og = _render_through_wrapper(ours, sc, cam, S, bg, cots)
-    assert oo["num_rendered"] == ro["num_rendered"]
-    assert torch.equal(oo["radii"], ro["radii"]) and torch.equal(oo["num_contrib"], ro["num_contrib"].to(oo["num_contrib"].dtype))
-    assert torch.equal(oo["visible"], ro["visible"])
-    for n in ("color", "opacity", "depth", "feature", "normal", "surface_xyz"):
-        assert (oo[n] - ro[n]).abs().max().item() <= 1e-4, n
+def test_dropin_wrapper_matches_reference_stock_path(P, W, H, S):
+    mod = dropin("r3dg_rasterization")
+    assert "relightable3dgaussian_b200" in mod._C.__file__
+    g = GoldenCase(REF_DROPIN, f"wrapper_{P}_{W}x{H}_S{S}")
+    sc, cam, bg, cots = wrapper_case(P, W, H, S)
+    oo, og = _render_through_wrapper(mod, sc, cam, S, bg, cots)
+    assert oo["num_rendered"] == int(g["num_rendered"])
+    for n in ("radii", "num_contrib", "visible"):
+        assert digest(oo[n]) == str(g[n]), n
+    for n in WRAPPER_IMAGES:
+        assert_close_to_summary(g, n, oo[n], max_abs=1e-4)
+    vis = np.nonzero(npy(oo["radii"]) > 0)[0]
     for n in og:
-        assert og[n] is not None and rg[n] is not None, n
-        assert rel_l2(npy(og[n]), npy(rg[n])) < 1e-3, n
+        assert og[n] is not None, n
+        assert_close_to_summary(g, "grad_" + n, og[n], rows=vis, rel=1e-3)
 
 
 def _bvh_scene(P):
@@ -77,61 +96,34 @@ def _bvh_scene(P):
     return d(sc.means3D), d(sc.scales), d(sc.rotations), d(sc.opacities[:, 0].contiguous()), d(sc.normals)
 
 
-def test_reference_raytracer_runs_unmodified_over_dropin():
-    ref_gpu = _need("bvh")
+def test_dropin_raytracer_matches_reference_raytracer():
     from oracle import oracle_sampling
-    ours = ref_gpu.load_reference_wrapper("bvh", "dropin")
-    theirs = ref_gpu.load_reference_wrapper("bvh", "ref")
-    xyz, s, r, op, nrm = _bvh_scene(30_000)
+    mod = dropin("bvh_tracing")
+    g = GoldenCase(REF_DROPIN, "raytracer")
+    xyz, s, r, op, nrm = _bvh_scene(RAYTRACER_P)
     icov = oracle_sampling.inverse_covariance(s, r)
-    a, b = ours.RayTracer(xyz, s, r), theirs.RayTracer(xyz, s, r)
-    for name in ("tree", "morton"):                                   # topology + Morton codes bit-exact
-        ta, tb = getattr(a, name, None), getattr(b, name, None)
-        if ta is not None and tb is not None:
-            assert torch.equal(ta, tb), name
+    a = mod.RayTracer(xyz, s, r)
+    assert digest(a.tree) == str(g["tree"]) and digest(a.morton) == str(g["morton"])   # topology + Morton codes bit-exact
     dirs, _ = oracle_sampling.sample_incident_rays(nrm, False, 24)
-    ro = xyz[:, None].expand_as(dirs)
-    va = a.trace_visibility(ro, dirs, xyz, icov, op, nrm)
-    vb = b.trace_visibility(ro, dirs, xyz, icov, op, nrm)
-    flips = ((va["visibility"] == 0) != (vb["visibility"] == 0)).float().mean().item()
-    same = (va["visibility"] == 0) == (vb["visibility"] == 0)
-    assert flips <= 1e-3, flips
-    assert (va["visibility"] - vb["visibility"])[same].abs().max().item() <= 1e-4
+    va = a.trace_visibility(xyz[:, None].expand_as(dirs), dirs, xyz, icov, op, nrm)
+    assert_visibility_close(g, "vis", va["visibility"], max_flips=1e-3, max_abs=1e-4)
 
 
 def test_sampling_kernel_vs_reference_function():
-    """r3dg_sample_incident_dirs vs the reference's own fibonacci_sphere_sampling (utils/graphics_utils.py:9-37, loaded
-    from the git-ignored copy) on this GPU, deterministic and random-rotate variants."""
-    ref_gpu = _need("bvh")
-    import importlib.util
-    import os
-    import sys
+    """r3dg_sample_incident_dirs vs the reference's own fibonacci_sphere_sampling (utils/graphics_utils.py:9-37) run on
+    a B200, deterministic and random-rotate variants."""
     from relightable3dgaussian_b200 import raytracer
-    py = os.path.join(os.path.dirname(ref_gpu.__file__), "_ref", "py")
-    sys.path.insert(0, py)
-    try:
-        saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "utils" or k.startswith("utils.")}
-        from utils.graphics_utils import fibonacci_sphere_sampling as ref_fib
-    finally:
-        sys.path.remove(py)
-        for k in [k for k in sys.modules if k == "utils" or k.startswith("utils.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-    g = torch.Generator().manual_seed(1)
-    nrm = torch.nn.functional.normalize(torch.randn(50_000, 3, generator=g), dim=-1).cuda()
-    nrm[0] = torch.tensor([0.0, 0.0, -1.0]); nrm[1] = torch.tensor([0.0, 0.0, 1.0])      # the -I fallback and the identity
-    for N in (24, 32, 384):
-        d_ref, a_ref = ref_fib(nrm, N, random_rotate=False)
+    g = GoldenCase(REF_DROPIN, "sampling")
+    nrm = sampling_normals()
+    for N in SAMPLING_N:
         d, a = raytracer.sample_incident_rays(nrm, False, N)
-        assert d.shape == d_ref.shape and a.shape == a_ref.shape and torch.equal(a, a_ref)
-        assert (d - d_ref).abs().max().item() <= 5e-7, N                                      # unit vectors: a few ulp at most
-        print(f"[sampling] N={N}: bit-equal fraction {(d == d_ref).float().mean().item():.6f}")
+        assert tuple(d.shape) == tuple(g[f"dirs_{N}_shape"]) and tuple(a.shape) == tuple(g[f"areas_{N}_shape"])
+        assert digest(npy(a).view(np.int32)) == str(g[f"areas_{N}"])
+        assert np.abs(spread(d, k=4096) - g[f"dirs_{N}"]).max() <= 5e-7, N                   # unit vectors: a few ulp at most
     # random rotation: same phase numbers through both
     torch.manual_seed(5)
-    d_ref, _ = ref_fib(nrm, 32, random_rotate=True)
-    torch.manual_seed(5)
     d, _ = raytracer.fibonacci_sphere_sampling(nrm, 32, random_rotate=True)
-    assert (d - d_ref).abs().max().item() <= 5e-6
+    assert np.abs(spread(d, k=4096) - g["dirs_rot"]).max() <= 5e-6
 
 
 @pytest.mark.parametrize("P,N", [(100_000, 32), (40_000, 64)])
@@ -139,18 +131,15 @@ def test_full_bake_parity_own_tree_vs_reference_tree(P, N):
     """update_visibility end to end: OUR tree (exact refit) + in-kernel sampling + our trace, against the REFERENCE's
     bake (its racy-refit tree, PyTorch sampling, its trace kernel, its chunk loop).  Visibility is a step function of T
     at 0.9, so the flip rate across that cliff is the meaningful figure (north_star)."""
-    ref_gpu = _need("bvh")
     from oracle import oracle_sampling
     from relightable3dgaussian_b200 import raytracer
+    g = GoldenCase(REF_DROPIN, f"bake_{P}_{N}")
     xyz, s, r, op, nrm = _bvh_scene(P)
     icov = oracle_sampling.inverse_covariance(s, r)
     assert (raytracer.inverse_covariance(s, r) - icov).abs().max().item() <= 1e-3 * icov.abs().max().item()
     vis, dirs, areas = raytracer.update_visibility(xyz, s, r, icov, op, nrm, N)
-    rvis, rdirs, rareas, _ = ref_gpu.reference_update_visibility(xyz, s, r, icov, op, nrm, N)
-    assert vis.shape == rvis.shape == (P, N, 1) and dirs.shape == rdirs.shape and torch.equal(areas, rareas)
-    assert (dirs - rdirs).abs().max().item() <= 5e-7
-    flip = ((vis == 0) != (rvis == 0)).float().mean().item()
-    same = (vis == 0) == (rvis == 0)
-    print(f"[bake] P={P} N={N}: blocked {float((rvis == 0).float().mean()):.3f}, flip rate {flip:.2e}, max-abs on agreeing rays {(vis - rvis)[same].abs().max().item():.2e}")
-    assert flip <= 1e-3
-    assert (vis - rvis)[same].abs().max().item() <= 1e-4
+    assert tuple(vis.shape) == tuple(g["vis_shape"]) == (P, N, 1) and dirs.shape == (P, N, 3)
+    assert digest(npy(areas).view(np.int32)) == str(g["areas"])
+    assert np.abs(spread(dirs, k=4096) - g["dirs"]).max() <= 5e-7
+    flip, err = assert_visibility_close(g, "vis", vis, max_flips=1e-3, max_abs=1e-4)
+    print(f"[bake] P={P} N={N}: flip rate {flip:.2e} (every 8th Gaussian), max-abs on agreeing sampled rays {err:.2e}")

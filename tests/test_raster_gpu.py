@@ -1,6 +1,6 @@
 """GPU parity tests (run on the B200 box: `pytest -m gpu`).  Everything goes through the C ABI of
-libr3dg_b200.so via the reference-shaped host API; the CPU oracle and, when its build travelled
-with the snapshot, the unmodified reference CUDA kernels (oracle/_ref) are the checkers.
+libr3dg_b200.so via the reference-shaped host API; the CPU oracle and outputs of the unmodified
+reference CUDA kernels stored under tests/golden/ are the checkers.
 
 Tolerances (BASELINE.json north_star): images <= 1e-4 max-abs, gradients <= 1e-3 relative,
 tile / sort indices bit-exact."""
@@ -12,7 +12,8 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import GOLDEN, ROOT, case_inputs, max_rel_above_floor, npy, oracle_kwargs, rel_l2
+from helpers import (GOLDEN, ROOT, GoldenCase, assert_close_to_summary, case_inputs, digest, max_rel_above_floor, npy,
+                     oracle_kwargs, rel_l2)
 
 pytestmark = pytest.mark.gpu
 RASTER_CASES = sorted(glob.glob(os.path.join(GOLDEN, "raster_*.npz")))
@@ -175,47 +176,57 @@ def test_matches_cpu_oracle_midsize(C, S, pseudo):
             assert rel_l2(npy(o["grads"][n]), gr[n]) < 1e-3, n
 
 
-def _live_reference_parity(C, P, W, H, S, view, center_shift, backward=True, recipe="shell-v1", sh_degree=3, M=16, scale_boost=1.0):
-    """Our kernels vs the UNMODIFIED reference kernels (oracle/_ref) on the same inputs, on this GPU:
-    tile / sort indices bit-exact, images <= 1e-4 max-abs, all nine gradients <= 1e-3 relative (north_star)."""
-    from oracle import ref_gpu
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref/libref_raster.so not present")
+REF_PARITY = os.path.join(GOLDEN, "refparity_raster.npz")
+PARITY_INDICES = ("radii", "tiles_touched", "point_list", "point_list_keys", "ranges", "n_contrib")
+PARITY_IMAGES = ("color", "opacity", "depth", "feature", "normal", "surface_xyz")
+
+
+def parity_inputs(P, W, H, S, view, center_shift, backward=True, recipe="shell-v1", sh_degree=3, M=16, scale_boost=1.0):
+    """One seeded comparison with the unmodified reference kernels: (case key, rasterizer kwargs, cotangents or None)."""
     sc, cam = case_inputs(P, W, H, S, view=view, center_shift=center_shift, recipe=recipe, scale_boost=scale_boost)
-    bg = torch.tensor([0.0, 0.5, 1.0])
-    kw = oracle_kwargs(sc, cam, bg)
-    extra = dict(shs=np.ascontiguousarray(npy(sc.shs)[:, :M]), scales=npy(sc.scales), rotations=npy(sc.rotations),
-                 features=npy(sc.features) if S else None, sh_degree=sh_degree)
+    kw = oracle_kwargs(sc, cam, torch.tensor([0.0, 0.5, 1.0]))
+    kw.update(shs=np.ascontiguousarray(npy(sc.shs)[:, :M]), scales=npy(sc.scales), rotations=npy(sc.rotations),
+              features=npy(sc.features) if S else None, sh_degree=sh_degree)
     g = torch.Generator().manual_seed(2)
     cots = [torch.randn(c, H, W, generator=g) for c in (3, 1, 1, S)] if backward else None
-    o = run_ours(C, cots=cots, **kw, **extra)
-    ref = ref_gpu.RefRasterizer()
-    tk = {k: (dev(v) if isinstance(v, np.ndarray) else v) for k, v in {**kw, **extra}.items() if v is not None}
-    ro = ref.forward(**tk)
-    assert o["num_rendered"] == ro["num_rendered"]
-    assert torch.equal(o["radii"], ro["radii"])
-    assert torch.equal(o["mid"]("tiles_touched"), ref.intermediate("tiles_touched"))
-    assert torch.equal(o["mid"]("point_list"), ref.intermediate("point_list"))
-    assert torch.equal(o["mid"]("point_list_keys"), ref.intermediate("point_list_keys"))
-    assert torch.equal(o["mid"]("ranges"), ref.intermediate("ranges")[: o["mid"]("ranges").shape[0]])
-    assert torch.equal(o["n_contrib"].reshape(-1), ref.intermediate("n_contrib"))
-    for n in ("color", "opacity", "depth", "feature", "normal", "surface_xyz"):
-        if ro[n].numel():
-            assert (o[n] - ro[n]).abs().max().item() <= 1e-4, n
-    assert (o["weights"] - ro["weights"]).abs().max().item() <= 1e-3 * max(1.0, ro["weights"].abs().max().item())
-    if backward:
-        rg = ref.backward(ro, dL_dcolor=dev(cots[0]), dL_dopacity=dev(cots[1]), dL_ddepth=dev(cots[2]), dL_dfeature=dev(cots[3]),
-                          **{k: v for k, v in tk.items() if k in ("means3D", "viewmatrix", "projmatrix", "campos", "bg",
-                                                                  "tan_fovx", "tan_fovy", "shs", "scales", "rotations", "features", "sh_degree")})
-        for n in GRADS:
-            if rg[n].numel() and float(rg[n].abs().max()) > 0:
-                assert rel_l2(npy(o["grads"][n]), npy(rg[n])) < 1e-3, n
-    del ref
-    torch.cuda.empty_cache()
+    key = f"{recipe}_{P}_{W}x{H}_S{S}_v{view}{'c' if center_shift else ''}_deg{sh_degree}M{M}_b{scale_boost:g}{'' if backward else '_fwd'}"
+    return key, kw, cots
+
+
+def parity_outputs(o, grads, W, H):
+    """The arrays a comparison with the reference looks at, from a forward dict (intermediates through o["mid"]) and
+    the gradient dict (None: forward only)."""
+    T = ((W + 15) // 16) * ((H + 15) // 16)
+    out = {n: o["mid"](n) for n in ("tiles_touched", "point_list", "point_list_keys")}
+    out.update(radii=o["radii"], ranges=o["mid"]("ranges")[:T], n_contrib=o["n_contrib"].reshape(-1), weights=o["weights"],
+               **{n: o[n] for n in PARITY_IMAGES}, **{"grad_" + n: t for n, t in (grads or {}).items()})
+    return out
+
+
+def _reference_parity(C, *case, **kwcase):
+    """Our kernels vs the UNMODIFIED reference kernels on the same inputs (tests/golden/refparity_raster.npz, made by
+    make_golden_refparity.py): tile / sort indices bit-exact (sha256 of the whole arrays), images <= 1e-4 max-abs,
+    all nine gradients <= 1e-3 relative (north_star), on a fixed sample of each array plus its full L2 norm."""
+    key, kw, cots = parity_inputs(*case, **kwcase)
+    g = GoldenCase(REF_PARITY, key)
+    o = run_ours(C, cots=cots, **kw)
+    got = parity_outputs(o, o.get("grads"), kw["W"], kw["H"])
+    assert o["num_rendered"] == int(g["num_rendered"])
+    for n in PARITY_INDICES:
+        assert digest(got[n]) == str(g[n]), n
+    vis = np.nonzero(npy(o["radii"]) > 0)[0]
+    for n in PARITY_IMAGES:
+        if n in g:
+            assert_close_to_summary(g, n, got[n], max_abs=1e-4)
+    assert_close_to_summary(g, "weights", got["weights"], rows=vis, max_abs=1e-3 * max(1.0, float(g["weights_maxabs"])))
+    for n in GRADS:
+        if "grad_" + n in g:
+            assert_close_to_summary(g, "grad_" + n, got["grad_" + n], rows=vis, rel=1e-3)
+    assert (cots is not None) == any("grad_" + n in g for n in GRADS)
 
 
 def test_matches_live_reference_kernels_if_built(C):
-    _live_reference_parity(C, 200_000, 640, 480, 5, view=5, center_shift=True)
+    _reference_parity(C, 200_000, 640, 480, 5, view=5, center_shift=True)
 
 
 @pytest.mark.parametrize("P,W,H,S,view,shift,bwd", [
@@ -226,21 +237,21 @@ def test_matches_live_reference_kernels_if_built(C):
     (2_000_000, 1920, 1080, 16, 6, False, True),    # BASELINE config #5 raster shape
 ], ids=["cfg2-300k-fwd", "cfg3-300k-fwdbwd", "headline-1M-S5", "cfg4-1.5M-1600x1200-S16", "cfg5-2M-1080p-S16"])
 def test_live_reference_parity_at_benchmark_sizes(C, P, W, H, S, view, shift, bwd):
-    _live_reference_parity(C, P, W, H, S, view, shift, backward=bwd)
+    _reference_parity(C, P, W, H, S, view, shift, backward=bwd)
 
 
 @pytest.mark.parametrize("S", [1, 3, 7, 9, 12, 13, 17, 20, 21, 24, 28, 33])
 def test_every_channel_group_instantiation(C, S):
     """The compositors are templates on the number of 4-channel groups (S = 0..33 forward, 0..24 backward, the
     reference's limits forward.cu:312 / backward.cu:449): every instantiation against the reference kernels."""
-    _live_reference_parity(C, 6_000, 208, 144, S, view=S % 8, center_shift=bool(S & 1), backward=S <= 24, scale_boost=2.0)
+    _reference_parity(C, 6_000, 208, 144, S, view=S % 8, center_shift=bool(S & 1), backward=S <= 24, scale_boost=2.0)
 
 
 @pytest.mark.parametrize("deg,M", [(0, 1), (1, 4), (2, 9), (3, 16), (1, 16), (0, 16)])
 def test_sh_degrees_and_row_widths(C, deg, M):
     """SH rows of 12 / 48 / 108 / 192 bytes: the bulk-copy slab path needs 16-byte rows, the others take the
     transposed LDGSTS path (projection.cu); degrees below the stored width ignore the upper coefficients."""
-    _live_reference_parity(C, 9_000, 200, 136, 5, view=deg + 2, center_shift=False, sh_degree=deg, M=M, scale_boost=1.5)
+    _reference_parity(C, 9_000, 200, 136, 5, view=deg + 2, center_shift=False, sh_degree=deg, M=M, scale_boost=1.5)
 
 
 def test_backward_launch_order_follows_measured_forward_work(C):
@@ -466,7 +477,8 @@ def test_bulk_copy_record_staging_variant_is_bit_identical(C):
             _lib.tune("composite_bulk", prev)
         for n in ("color", "opacity", "depth", "feature", "n_contrib", "normal"):
             assert torch.equal(a[n], b[n]), n
-        assert (a["weights"] - b["weights"]).abs().max().item() < 1e-5
+        # weights are accumulated with float atomics, so two runs differ in the last bits of the larger values
+        assert bool(((a["weights"] - b["weights"]).abs() < 1e-5 * b["weights"].abs().clamp_min(1.0)).all())
     sc, cam = case_inputs(300_000, 800, 800, 16, view=1)
     kw = oracle_kwargs(sc, cam, torch.tensor([0.0, 0.5, 1.0]))
     extra = dict(shs=npy(sc.shs), scales=npy(sc.scales), rotations=npy(sc.rotations), features=npy(sc.features))
